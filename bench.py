@@ -5,7 +5,7 @@
     python bench.py --impl reference --gpus N --steps K --warmup W
 
 Front door: the REAL ``modin.pandas`` with this repo's execution plugged in (``modin_b200.modin_plugin``;
-Modin itself comes from ``baseline/_ref``, pip-installed from the read-only reference) -- ``config.api`` says so.
+Modin itself comes from ``oracle/_ref``, which ``build()`` installs from the original project) -- ``config.api`` says so.
 ``--api mirror`` (and the automatic fallback when Modin is not importable) uses the repo's own Modin-free mirror
 of the same class protocol, ``modin_b200.pandas``.
 
@@ -27,7 +27,12 @@ One JSON line on rank 0:
   every leg carries ``checked`` (its result was verified OUTSIDE the timed region); N > 1 adds ``parity_ok``
   (the hot path checked against pandas on a small job-wide frame over the NCCL group before anything is timed).
 
-``--impl reference`` times the UNMODIFIED reference (``modin.pandas`` from ``baseline/_ref``, its own
+``--dump-outputs DIR`` writes what the timed steps of each leg computed in their last step as ``DIR/<name>.npy``
+(float64; rows of large results at fixed seeded positions, with those positions as ``<name>_rows`` / ``<name>_index``),
+so that two builds can be compared output for output on identical inputs.  Groupby sums accumulate with float
+atomics and match from run to run only within the sum tolerance; every other output repeats bit for bit.
+
+``--impl reference`` times the UNMODIFIED reference (``modin.pandas`` from ``oracle/_ref``, its own
 PandasOnPython engine -- PandasOnRay when ``ray`` is importable) on a bounded sample of the same workload; rank 0
 only.
 """
@@ -46,12 +51,16 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
-REF = os.path.join(ROOT, "baseline", "_ref")
+REF = os.path.join(ROOT, "oracle", "_ref")
 
 METRIC = "rows/sec elementwise map (a*b+c) on 1e9x8 f64"
 UNIT = "rows/s"
 B_SCALAR, C_SCALAR = 1.000000119, 0.5
 EPS = 2.0**-53
+# --dump-outputs: at most 3 MB per result (sampled values + their positions); the ten sampled results plus the two
+# 16-value reductions stay far below 64 MB whatever --cols is
+DUMP_BYTES_PER_OUTPUT = 3 << 20
+DUMP_SEED = 20_251_017
 
 
 def parse_args():
@@ -70,6 +79,8 @@ def parse_args():
     ap.add_argument("--skip-also", action="store_true")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write each leg's result of its last timed step to DIR/<name>.npy (rank 0's shard when N > 1)")
     return ap.parse_args()
 
 
@@ -94,6 +105,18 @@ def traffic_for(kernel: str, rows_local: int = 0):
         return None
 
 
+def dump_positions(n: int, ncols: int):
+    """Rows kept of an n-row, ncols-column result: all of them when they fit DUMP_BYTES_PER_OUTPUT, else the first and
+    the last row and a seeded draw -- the same positions for the same shape in every run."""
+    import numpy as np
+
+    k = max(2, DUMP_BYTES_PER_OUTPUT // (8 * (ncols + 1)))
+    if n <= k:
+        return np.arange(n, dtype=np.int64)
+    draw = np.random.default_rng(DUMP_SEED).integers(0, n, k - 2)
+    return np.unique(np.concatenate([np.array([0, n - 1], dtype=np.int64), draw]))
+
+
 def modin_importable() -> bool:
     return os.path.isdir(os.path.join(REF, "modin"))
 
@@ -109,7 +132,7 @@ _MALLOC_ENV = {
 
 
 def _reference_modin():
-    """``modin.pandas`` of the UNMODIFIED reference (baseline/_ref) on its own CPU engine; (module, engine name)."""
+    """``modin.pandas`` of the UNMODIFIED reference (oracle/_ref) on its own CPU engine; (module, engine name)."""
     if REF not in sys.path:
         sys.path.insert(0, REF)
     from modin_b200.modin_plugin import apply_pandas3_shims
@@ -144,7 +167,7 @@ def run_reference_arm(args):
 
     ncpu = os.cpu_count() or 1
     if not modin_importable():
-        print(json.dumps({"impl": "reference", "unavailable": "baseline/_ref/modin is not installed on this box"}), flush=True)
+        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/modin is not installed on this box"}), flush=True)
         return
     mpd, engine, nparts = _reference_modin()
     cores = 1 if engine == "PandasOnPython" else ncpu
@@ -209,7 +232,7 @@ def run_reference_arm(args):
         "config": {"workload": f"map_partitions elementwise a*b+c (b,c scalars) on {int(args.rows)}x{W} f64 -- reference "
                                f"arm: a {rows}x{W} sample of it per step",
                    "rows": int(args.rows), "cols": W, "sample_rows": rows,
-                   "api": f"modin.pandas ({engine}, unmodified reference from baseline/_ref, pandas-3 import shims)",
+                   "api": f"modin.pandas ({engine}, unmodified reference from oracle/_ref, pandas-3 import shims)",
                    "npartitions": nparts},
         "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": "reference", "engine": engine,
                          "host_cores": ncpu,
@@ -305,7 +328,7 @@ class Api:
 
             cfg.NPartitions.put(1)
             self.pd = mpd
-            self.name = "modin.pandas (ArrowOnB200: real Modin from baseline/_ref + modin_b200.modin_plugin)"
+            self.name = "modin.pandas (ArrowOnB200: real Modin from oracle/_ref + modin_b200.modin_plugin)"
         else:
             import modin_b200.pandas as bpd
 
@@ -335,6 +358,12 @@ class Api:
         if qc is not None:
             qc.finalize()
         return obj
+
+    def cumsum(self, obj):
+        """``df.cumsum()``; the mirror's API layer has no Fold methods, so there the query compiler's is called."""
+        if self.which == "modin":
+            return obj.cumsum()
+        return self.pd.DataFrame(query_compiler=obj._query_compiler.cumsum(0))
 
     @staticmethod
     def to_pandas(obj):
@@ -528,6 +557,27 @@ def run_b200_arm(args):
     def device_values(col, idx):
         return col.data[torch.tensor(idx, dtype=torch.int64, device=col.data.device)].cpu().numpy()
 
+    dumped = {}  # --dump-outputs: name -> float64 array, kept on rank 0 and written after the last leg
+
+    def dump(name, arr):
+        if args.dump_outputs is not None and rank == 0:
+            dumped[name] = np.asarray(arr, dtype=np.float64)
+
+    def dump_block(name, frame, row0):
+        """Sampled rows of this rank's device result block of ``frame``, and their positions in the whole frame."""
+        if args.dump_outputs is not None and rank == 0:
+            blk = api.blocks(frame)[0]
+            idx = dump_positions(blk.nrows, len(blk.cols))
+            dump(name, np.stack([device_values(c, idx) for c in blk.cols], axis=1))
+            dump(name + "_rows", idx + row0)
+
+    def dump_frame(name, frame):
+        """Sampled rows of a host result frame, and its index at those rows."""
+        if args.dump_outputs is not None and rank == 0:
+            idx = dump_positions(len(frame), frame.shape[1])
+            dump(name, frame.iloc[idx].to_numpy(dtype=np.float64))
+            dump(name + "_index", frame.index.to_numpy()[idx])
+
     # ---- multi-GPU parity before anything is timed ------------------------------------------------
     parity_ok, parity_fails = None, []
     progress(f"start: {ws} rank(s), {rows} rows, front door {api.which}")
@@ -556,6 +606,7 @@ def run_b200_arm(args):
     step_map()
     launches0 = lib.mb200_launch_count()
     total_ms, per = timed(step_map, args.steps, args.warmup)
+    dump_block("map_abc", last[0], lo)
     launches = lib.mb200_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
     launches_timed = round(launches * args.steps / max(args.steps + args.warmup, 1))
@@ -583,7 +634,7 @@ def run_b200_arm(args):
 
     def _secondary_legs():
         nonlocal a, roofline_groupby
-        ksteps = max(5, args.steps // 2)
+        ksteps = args.steps
         cols8 = [f"c{j}" for j in range(W)]
         # sums of the headline frame with the direct-load reduce kernel: the cross-check value for the TMA kernel below
         _cfg.ReduceVariant.put(1)
@@ -610,6 +661,7 @@ def run_b200_arm(args):
         for name, fn in (("sum", step_sum), ("mean", step_mean)):
             total_s, per_s = timed(fn, ksteps, 2)
             got = np.asarray(api.to_pandas(res[name]), dtype=np.float64)
+            dump(f"reduce_{name}", got)
             if name == "sum":
                 sum16 = got
                 ok = _sum_close(got[:W], sum8_ldg, abs8, rows)  # same first 8 columns, other reduce kernel
@@ -641,6 +693,7 @@ def run_b200_arm(args):
 
         total_f, per_f = timed(step_fma3, ksteps, 2)
         blk = api.blocks(last[0])[0]
+        dump_block("map_fma3", last[0], lo3)
         idx = sample_rows(blk.nrows)
         j = W - 1
         ref = (np.array([synth.gen_f64(1, 42, j, lo3 + r)[0] for r in idx]) * np.array([synth.gen_f64(1, 44, j, lo3 + r)[0] for r in idx])
@@ -664,10 +717,11 @@ def run_b200_arm(args):
 
             def step_cumsum():
                 last[0] = None
-                last[0] = api.launch(ff.cumsum())  # qc.cumsum -> Fold template -> frame.fold -> DevCumulative
+                last[0] = api.launch(api.cumsum(ff))  # qc.cumsum -> Fold template -> frame.fold -> DevCumulative
 
             total_c, per_c = timed(step_cumsum, ksteps, 2)
             blk = api.blocks(last[0])[0]
+            dump_block("fold_cumsum", last[0], lof)
             j = W - 1
             ok = True
             fsum = np.asarray(api.to_pandas(ff.sum()), dtype=np.float64)
@@ -696,7 +750,7 @@ def run_b200_arm(args):
         release()
 
         # ---- GroupByReduce: groupby('key').sum(), G int64 keys, 8 float64 values (C4)
-        def groupby_leg(skew, dense_on, label, kern, traffic_key):
+        def groupby_leg(skew, dense_on, label, kern, traffic_key, name):
             nonlocal roofline_groupby
             progress(f"leg: groupby{label or ' dense'}")
             g = api.device_frame(rows, W, seed=42, key_modulus=G, key_skew=skew)
@@ -715,7 +769,9 @@ def run_b200_arm(args):
 
             try:
                 total_g, per_g = timed(step_gb, ksteps, 2)
-                total_full, _ = timed(step_gb_full, 3, 1)
+                if args.dump_outputs is not None:  # on every rank: gathering the key ranges is collective
+                    dump_frame(name, api.to_pandas(last[0]))
+                total_full, _ = timed(step_gb_full, ksteps, 1)
                 k_ms = kernel_ms(step_gb, "gb_accumulate")
                 # ---- checks, outside the timed region
                 res = api.to_pandas(last[0])  # gathers every rank's key range: G x 8 (72 MB at G = 1e6)
@@ -744,7 +800,7 @@ def run_b200_arm(args):
                      "value": rows / (total_g / ksteps / 1e3), "unit": UNIT, "ms_per_step": total_g / ksteps,
                      "groups": int(len(keys)), "checked": ok, "roofline": rf,
                      "step": "gb = df.groupby('key') once; timed: gb.sum()",
-                     "ms_per_step_full_expression": total_full / 3}  # fmt: skip
+                     "ms_per_step_full_expression": total_full / ksteps}  # fmt: skip
             also.append(entry)
             if not skew and dense_on:
                 roofline_groupby = dict(rf, value=entry["value"], ms_per_step=entry["ms_per_step"], checked=ok,
@@ -753,9 +809,12 @@ def run_b200_arm(args):
             del g
             release()
 
-        groupby_leg(False, True, "", "gb_accumulate_tma_kernel on a dense (direct-addressed) table pinned in L2", "groupby_sum_dense")
-        groupby_leg(False, False, " [hash table forced]", "gb_accumulate_tma_kernel (open-addressed hash aggregate)", "groupby_sum")
-        groupby_leg(True, True, " SKEWED (Zipf-like)", "gb_accumulate_tma_kernel<HOT> (dense table, per-CTA hot-group cache)", None)
+        groupby_leg(False, True, "", "gb_accumulate_tma_kernel on a dense (direct-addressed) table pinned in L2", "groupby_sum_dense",
+                    "groupby_sum_dense")
+        groupby_leg(False, False, " [hash table forced]", "gb_accumulate_tma_kernel (open-addressed hash aggregate)", "groupby_sum",
+                    "groupby_sum_hash")
+        groupby_leg(True, True, " SKEWED (Zipf-like)", "gb_accumulate_tma_kernel<HOT> (dense table, per-CTA hot-group cache)", None,
+                    "groupby_sum_skewed")
         # what a key column of UNKNOWN origin pays once: the 8 B/row statistics pass (mb200_key_range)
         from modin_b200 import ops as _ops
 
@@ -796,6 +855,7 @@ def run_b200_arm(args):
                 os.environ["MB200_JOIN_DENSE"] = "0"
             try:
                 total_m, per_m = timed(step_merge, ksteps, 2)
+                dump_block("merge_left_" + ("dense" if dense_on else "hash"), last[0], lo)
                 km_ms = kernel_ms(step_merge, "join_probe_gather")
             finally:
                 os.environ.pop("MB200_JOIN_DENSE", None)
@@ -849,14 +909,14 @@ def run_b200_arm(args):
             m = min(len(arr), 1 << 20)
             arr[:] = np.resize(synth.gen_f64(m, seed, col), len(arr))
 
-        def host_timed(step_fn, reps=3):
+        def host_timed(step_fn):
             step_fn()
             sync_all()
             t0 = time.perf_counter()
-            for _ in range(reps):
+            for _ in range(args.steps):
                 step_fn()
             torch.cuda.synchronize()
-            return max_over_ranks((time.perf_counter() - t0) / reps * 1e3)
+            return max_over_ranks((time.perf_counter() - t0) / args.steps * 1e3)
 
         with dist.local_frames():  # every rank runs the same host-to-host pipeline on ITS OWN host frame
             try:
@@ -873,6 +933,7 @@ def run_b200_arm(args):
 
                 dt = host_timed(step_e2e)
                 got = out[0]
+                dump_frame("e2e_map_abc", got)
                 ref = host["c0"].to_numpy()[:1000] * B_SCALAR + C_SCALAR
                 ok = got.shape == (er, W) and bool((got["c0"].to_numpy()[:1000] == ref).all()) and \
                     bool((got[f"c{W - 1}"].to_numpy()[-1000:] == host[f"c{W - 1}"].to_numpy()[-1000:] * B_SCALAR + C_SCALAR).all())
@@ -897,8 +958,9 @@ def run_b200_arm(args):
                     df = api.pd.DataFrame(host)
                     out[0] = api.to_pandas(df.groupby("key").sum())  # H2D 72 B/row, device groupby, result D2H
 
-                dt = host_timed(step_e2e_gb, reps=2)
+                dt = host_timed(step_e2e_gb)
                 got = out[0]
+                dump_frame("e2e_groupby_sum", got)
                 keys = host["key"].to_numpy()
                 ok = len(got) == len(np.unique(keys[: 1 << 22])) if er >= (1 << 22) else True
                 want0 = np.bincount(keys, weights=host["c0"].to_numpy(), minlength=G)[got.index.to_numpy()]
@@ -932,6 +994,10 @@ def run_b200_arm(args):
             cpu = {"value": None, "unit": UNIT, "cores": 0, "kind": "reference", "sample": f"failed: {e!r}"[:300]}
 
     progress("done")
+    if args.dump_outputs is not None and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     if rank == 0:
         line = {
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": ws, "steps": args.steps,

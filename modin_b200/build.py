@@ -1,7 +1,7 @@
 """In-tree build of libmodin_b200.so (sm_100a only) with plain nvcc.
 
 ``python -m modin_b200.build`` or ``__graft_entry__.build()``.  The shared library lands in
-``modin_b200/_native/`` (git-ignored, but it travels with the gpurun snapshot).  There is a
+``modin_b200/_native/`` (git-ignored, like the build stamp next to it).  There is a
 single code target -- ``-gencode arch=compute_100a,code=sm_100a`` -- and no fallback build.
 """
 
@@ -47,8 +47,8 @@ def _digest() -> str:
     h = hashlib.sha256()
     files = sources() + sorted(os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith(".cuh"))
     files.append(os.path.join(INCLUDE, "modin_b200.h"))
-    for f in files:
-        h.update(f.encode())
+    for f in files:  # names relative to the checkout: the same tree gives the same stamp wherever it lives
+        h.update(os.path.relpath(f, os.path.dirname(HERE)).encode())
         with open(f, "rb") as fh:
             h.update(fh.read())
     h.update(" ".join(NVCC_FLAGS).encode())

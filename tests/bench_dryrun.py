@@ -1,5 +1,5 @@
 """Dry run of ``bench.py``'s GPU arm on a box WITHOUT GPUs: the same function (``bench.run_b200_arm``), the same front
-door (real ``modin.pandas`` + plug-in when baseline/_ref is installed), the same legs, checks and collectives -- on the
+door (real ``modin.pandas`` + plug-in when oracle/_ref is installed), the same legs, checks and collectives -- on the
 numpy device double (tests/cpu_double.py), under gloo, with ``torch.cuda.*`` replaced by host stand-ins and tiny frames.
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29655 \

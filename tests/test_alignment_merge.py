@@ -17,7 +17,7 @@ from modin_b200 import synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REF = os.path.join(ROOT, "baseline", "_ref")
+REF = os.path.join(ROOT, "oracle", "_ref")
 
 
 def _same(got, want, what):
@@ -129,7 +129,7 @@ def _modin(nparts=4):
     return mpd
 
 
-needs_modin = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "modin")), reason="reference Modin not installed under baseline/_ref")
+needs_modin = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "modin")), reason="reference Modin not installed under oracle/_ref")
 
 
 @needs_modin

@@ -174,7 +174,7 @@ def test_fold_and_reduce_through_real_modin():
     from tests.test_alignment_merge import REF, _modin
 
     if not os.path.isdir(os.path.join(REF, "modin")):
-        pytest.skip("baseline/_ref (the unmodified reference) is not installed on this box")
+        pytest.skip("oracle/_ref (the unmodified reference) is not installed on this box")
     _front_door_checks(_modin(nparts=1), True)
 
 

@@ -3,7 +3,7 @@ in behind ``modin.pandas`` and the hot-path operations run through Modin's own A
 compiler caster, operator templates and ``PandasDataframe`` methods into this package's partition
 classes and device functors.
 
-Modin comes from ``baseline/_ref`` (pip-installed from the read-only reference, git-ignored; it
+Modin comes from ``oracle/_ref`` (installed by ``build()`` from the original project, git-ignored; it
 travels to the GPU box with the snapshot).  Without it these tests are skipped.  On a box without a
 GPU the device is the numpy test double (host logic only); the ``gpu``-marked variant at the bottom
 runs the same scenarios on the B200.
@@ -20,10 +20,10 @@ from modin_b200 import synth
 from oracle import reference_path as orc
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "baseline", "_ref")
+REF = os.path.join(ROOT, "oracle", "_ref")
 
 pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "modin")),
-                                reason="reference Modin not installed under baseline/_ref")  # fmt: skip
+                                reason="reference Modin not installed under oracle/_ref")  # fmt: skip
 
 
 def _same(a, b):

@@ -295,16 +295,16 @@ def test_third_batch_vs_reference_golden(golden_dir):
 def test_late_additions_under_real_modin_on_b200():
     """The same astype / drop_duplicates / unique / concat / nunique / reset_index scenarios as
     tests/test_modin_plugin.py::test_late_additions_under_real_modin_cpu_double, through real ``modin.pandas`` with
-    the B200 execution plugged in.  Needs the reference Modin under baseline/_ref (it travels with the snapshot)."""
+    the B200 execution plugged in.  Needs the reference Modin under oracle/_ref (it travels with the snapshot)."""
     import importlib.util
     import os
     import sys
     import warnings
 
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    ref = os.path.join(root, "baseline", "_ref")
+    ref = os.path.join(root, "oracle", "_ref")
     if not os.path.isdir(os.path.join(ref, "modin")):
-        pytest.skip("reference Modin not installed under baseline/_ref")
+        pytest.skip("reference Modin not installed under oracle/_ref")
     if ref not in sys.path:
         sys.path.insert(0, ref)
     warnings.filterwarnings("ignore")

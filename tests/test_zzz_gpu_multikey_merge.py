@@ -33,7 +33,7 @@ def test_multi_key_merge_on_b200():
 @UNTRIED
 def test_float_key_groupby_on_b200():
     if not os.path.isdir(os.path.join(REF, "modin")):
-        pytest.skip("baseline/_ref (the unmodified reference) is not installed on this box")
+        pytest.skip("oracle/_ref (the unmodified reference) is not installed on this box")
     _seventh_batch_checks(_modin())
 
 
@@ -41,7 +41,7 @@ def test_float_key_groupby_on_b200():
 @UNTRIED
 def test_groupby_level_on_b200():
     if not os.path.isdir(os.path.join(REF, "modin")):
-        pytest.skip("baseline/_ref (the unmodified reference) is not installed on this box")
+        pytest.skip("oracle/_ref (the unmodified reference) is not installed on this box")
     from tests.test_modin_plugin import _level_scenarios
 
     _level_scenarios(_modin())

@@ -8,7 +8,7 @@ rank), runs the hot-path templates through the public API and compares the gathe
 the CPU oracle.  Exit code 0 = all checks passed on every rank.
 
 ``--api mirror`` (default: both) drives ``modin_b200.pandas``; ``--api modin`` drives the REAL ``modin.pandas``
-(baseline/_ref) with the plug-in activated on every rank -- the same checks, plus the operations the plug-in refuses
+(oracle/_ref) with the plug-in activated on every rank -- the same checks, plus the operations the plug-in refuses
 on all ranks together.
 """
 import math
@@ -46,7 +46,7 @@ def front_door(which):
         import modin_b200.pandas as bpd
 
         return bpd
-    ref = os.path.join(ROOT, "baseline", "_ref")
+    ref = os.path.join(ROOT, "oracle", "_ref")
     if ref not in sys.path:
         sys.path.insert(0, ref)
     import warnings
@@ -178,10 +178,10 @@ def main():
     config.NPartitions.put(2)
     fails = []
     apis = ["mirror", "modin"] if args.api == "both" else [args.api]
-    if "modin" in apis and not os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "modin")):
+    if "modin" in apis and not os.path.isdir(os.path.join(ROOT, "oracle", "_ref", "modin")):
         apis.remove("modin")
         if rank == 0:
-            print("SKIP modin front door: baseline/_ref/modin is not installed", flush=True)
+            print("SKIP modin front door: oracle/_ref/modin is not installed", flush=True)
     for which in apis:
         try:
             run_checks(front_door(which), which, rank, fails)
